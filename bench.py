@@ -2,6 +2,7 @@
 """Benchmark of the ALIGNN edge-gated conv hot path on B200 (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--norm batchnorm|layernorm]
+                    [--dump-outputs DIR]
 
 A "step" is one forward + backward + optimizer update of ALIGNN (4 ALIGNN + 4 GCN layers, hidden
 256, the `ALIGNN` class of alignn/models/alignn.py, L1 loss as in train.py:240) on one synthetic
@@ -15,6 +16,11 @@ Prints ONE JSON line (rank 0).  Keys follow the driver contract; extra keys:
   e2e           same metric with the batch starting in pinned HOST memory every step and the loss read back
 `--impl reference` times that CPU oracle alone (the reference's own implementation needs DGL, which
 cannot be installed offline; see DESIGN.md).
+`--dump-outputs DIR` writes what the last timed step of `value` returned as float32 .npy files (rank 0): out.npy
+(predictions), loss.npy, grad.npy (the flat gradient buffer) and state.npy (every floating-point tensor of the model's
+state_dict after the optimizer update, flattened in state_dict order), 32 MB for the default model.  Inputs,
+initialisation and the number of steps before it are fixed by the arguments, so two builds run with the same
+arguments can be compared output for output.
 """
 import argparse
 import json
@@ -28,6 +34,7 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
+import numpy as np  # noqa: E402
 import torch  # noqa: E402
 import torch.distributed as dist  # noqa: E402
 
@@ -48,7 +55,13 @@ def parse():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-graph", action="store_true", help="launch every kernel eagerly instead of replaying CUDA graphs")
     ap.add_argument("--cpu-sample-graphs", type=int, default=0, help="0 = calibrate (~4 s of CPU work per step)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step to DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
+    return args
 
 
 # ---------------------------------------------------------------------------------------------
@@ -210,6 +223,14 @@ class ClockSampler:
                 "samples": len(sm)}
 
 
+def dump_outputs(directory, out, loss, grad, model):
+    """One step's predictions, loss, flat gradient buffer and resulting model state as float32 .npy files."""
+    os.makedirs(directory, exist_ok=True)
+    state = torch.cat([t.reshape(-1).float() for t in model.state_dict().values() if t.is_floating_point()])
+    for name, t in (("out", out), ("loss", loss), ("grad", grad), ("state", state)):
+        np.save(os.path.join(directory, name + ".npy"), t.detach().float().cpu().numpy())
+
+
 # ---------------------------------------------------------------------------------------------
 # our arm
 # ---------------------------------------------------------------------------------------------
@@ -263,7 +284,7 @@ def run_ours(args):
             loss.backward()
         reducer.all_reduce()
         opt.step()
-        return loss
+        return out, loss
 
     def h2d(i):
         g, lg, lat, tgt = host[i % nb]
@@ -285,39 +306,23 @@ def run_ours(args):
 
     def timed(fn, steps):
         """EXACTLY `steps` calls between two events on the launching stream, barrier + synchronize on both sides,
-        max over ranks."""
+        max over ranks.  Returns (ms, what the last call returned)."""
         barrier()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         with torch.cuda.stream(work):
             e0.record()
             for i in range(steps):
-                fn(i)
+                last = fn(i)
             e1.record()
         barrier()
         if world > 1 and cpu_group_ref[0] is not None:
             ms = torch.tensor([e0.elapsed_time(e1)])
             dist.all_reduce(ms, op=dist.ReduceOp.MAX, group=cpu_group_ref[0])
-            return ms.item()
+            return ms.item(), last
         ms = torch.tensor([e0.elapsed_time(e1)], device=dev)
         if world > 1:
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
-        return ms.item()
-
-    def timed_repeats(fn, steps, budget_s=2.5, max_reps=10):
-        """Median of up to `max_reps` repetitions of exactly `steps` steps (the clock sampler needs seconds, a 20-step
-        region lasts ~0.2 s); every repetition is a full timed region as above."""
-        first = timed(fn, steps)
-        reps = int(max(1, min(max_reps, budget_s * 1e3 / max(first, 1e-3))))
-        if world > 1:
-            if cpu_group_ref[0] is not None:
-                t = torch.tensor([reps])
-                dist.broadcast(t, 0, group=cpu_group_ref[0])
-            else:
-                t = torch.tensor([reps], device=dev)
-                dist.broadcast(t, 0)
-            reps = int(t.item())
-        all_ms = [first] + [timed(fn, steps) for _ in range(reps - 1)]
-        return statistics.median(all_ms), all_ms
+        return ms.item(), last
 
     # ---- warm-up (also builds the flat gradient buffer, the flat optimizer and the operand-image tables) ------------
     with torch.cuda.stream(work):
@@ -356,7 +361,7 @@ def run_ours(args):
         if nccl_in_graph:
             reducer.reduce_flat()
             opt.step()
-        return loss
+        return out, loss
 
     if use_graph:
         pool = None
@@ -364,10 +369,10 @@ def run_ours(args):
             gr = torch.cuda.CUDAGraph()
             l0 = _lib.launch_count()
             with torch.cuda.graph(gr, pool=pool, stream=work, capture_error_mode="thread_local" if nccl_in_graph else "global"):
-                loss_b = fwd_bwd(resident[b])
+                out_b, loss_b = fwd_bwd(resident[b])
             launches_per_step = _lib.launch_count() - l0
             pool = pool or gr.pool()
-            graphs_res.append((gr, loss_b))
+            graphs_res.append((gr, out_b, loss_b))
         if not nccl_in_graph:
             graph_opt = torch.cuda.CUDAGraph()
             l0 = _lib.launch_count()
@@ -377,13 +382,15 @@ def run_ours(args):
         barrier()
 
     def run_resident(i):
+        """One step on resident batch i % nb; returns (predictions, loss), valid until that batch's next step."""
         if use_graph:
-            graphs_res[i % nb][0].replay()
+            gr, out, loss = graphs_res[i % nb]
+            gr.replay()
             if not nccl_in_graph:
                 reducer.reduce_flat()
                 graph_opt.replay()
-        else:
-            step(resident[i % nb])
+            return out, loss
+        return step(resident[i % nb])
 
     # End to end = what a training loop with a prefetching loader does (train.py's DataLoader has pin_memory and
     # worker prefetch): while the GPU works on batch i, a copy stream moves batch i+1 from pinned host memory into the
@@ -413,12 +420,12 @@ def run_ours(args):
 
     def run_e2e(i):
         if not use_graph:
-            return step(h2d(i)).item()                        # D2H + sync, as train.py:300-305 does
+            return step(h2d(i))[1].item()                     # D2H + sync, as train.py:300-305 does
         b = i % nb
         if pf["slot_has"] != i:
             prefetch(i)                                       # nobody copied this step's inputs yet: do it now
         work.wait_event(copy_done[b])
-        gr, loss_b = graphs_res[b]
+        gr, _, loss_b = graphs_res[b]
         gr.replay()
         if not nccl_in_graph:
             reducer.reduce_flat()
@@ -441,14 +448,16 @@ def run_ours(args):
     if rank == 0:
         sampler.start()
     l0 = _lib.launch_count()
-    ms_total, reps_res = timed_repeats(run_resident, args.steps)
-    launches = (launches_per_step * args.steps) if use_graph else ((_lib.launch_count() - l0) // max(len(reps_res), 1))
+    ms_total, (out_last, loss_last) = timed(run_resident, args.steps)
+    launches = (launches_per_step * args.steps) if use_graph else (_lib.launch_count() - l0)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, out_last, loss_last, reducer.flat, model)
 
     # ---- timed: end to end from pinned host memory, loss read back every step ----------------
     with torch.cuda.stream(work):
         for i in range(2):
             run_e2e(i)
-    ms_e2e, reps_e2e = timed_repeats(run_e2e, args.steps)
+    ms_e2e, _ = timed(run_e2e, args.steps)
     clocks = sampler.stop() if rank == 0 else None
 
     # ---- per-kernel table: CUDA events around every library call in an eager replay of the same steps (events inside
@@ -457,7 +466,7 @@ def run_ours(args):
         for i in range(2):                                    # eager allocations settle on this stream
             step(resident[i % nb])
     ops.TIMER = ops.KernelTimer()
-    ms_eager = timed(lambda i: step(resident[i % nb]), args.steps)
+    ms_eager, _ = timed(lambda i: step(resident[i % nb]), args.steps)
     ksum = ops.TIMER.summary()
     ops.TIMER = None
 
@@ -514,15 +523,14 @@ def run_ours(args):
         "run": {"device": "B200", "N": N, "E": E, "T": T,
                 "optimizer_impl": "one launch over one flat parameter (alignn_b200.dp.FlatAdamW -> alignn_b200_adamw_flat)",
                 "cuda_graph": use_graph, "allreduce_in_graph": bool(nccl_in_graph), "eager_ms_per_step": ms_eager / args.steps,
-                "timing": f"median of {len(reps_res)} repetitions of exactly {args.steps} steps (each: events on the launching "
-                          f"stream, barrier + synchronize on both sides, max over ranks)",
-                "repetition_ms": [round(m, 3) for m in reps_res]},
+                "timing": f"exactly {args.steps} steps between two events on the launching stream, barrier + synchronize "
+                          f"on both sides, max over ranks"},
         "roofline": roofline,
         "step_hbm": {"algorithmic_bytes_per_step": sbytes, "achieved": sbytes / (ms_step * 1e-3) / 1e9, "peak": peak,
                      "unit": "GB/s", "frac": sbytes / (ms_step * 1e-3) / 1e9 / peak,
                      "note": "conv-stack compulsory bytes per batch (SURVEY 8d) / whole step time incl. embeddings, GEMMs, optimizer"},
         "e2e": {"value": e2e_value, "unit": UNIT, "ms_per_step": ms_e2e / args.steps,
-                "h2d_bytes_per_step": int(h2d_bytes), "d2h_bytes_per_step": 4, "repetition_ms": [round(m, 3) for m in reps_e2e],
+                "h2d_bytes_per_step": int(h2d_bytes), "d2h_bytes_per_step": 4,
                 "how": ("every step: inputs pinned host -> device (copy stream, issued one step ahead so it overlaps the previous step's "
                         "kernels; the first step of a region copies its own inputs serially), CUDA-graph replay, loss device -> pinned "
                         "host, read by the host one step later") if use_graph else

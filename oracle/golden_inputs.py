@@ -65,6 +65,16 @@ def checksum(*arrays) -> int:
     return c
 
 
+def sample(a, n: int = 4096) -> np.ndarray:
+    """A fixed subset of at most `n` elements of `a`: the flattened array at an odd stride, which visits every column
+    of the power-of-two-wide feature and weight matrices.  Large fixture arrays are stored as this sample (bounds the
+    file size); tests compare the same subset of what they compute."""
+    if isinstance(a, torch.Tensor):
+        a = a.detach().cpu().numpy()
+    a = np.asarray(a).reshape(-1)
+    return a[::max(1, -(-a.size // n)) | 1]
+
+
 # JVASP-98225 (32 atoms: 16 K + 16 Bi) cartesian coordinates are read by make_golden.py
 # from the reference test (alignn/tests/test_force_reduction.py:22-55) at generation time
 # and stored inside tests/golden/jvasp_98225.npz; tests read them from there.

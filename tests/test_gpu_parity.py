@@ -78,7 +78,7 @@ def test_conv_jvasp_vs_reference_golden(golden_dir, tag, norm, train):
     x, y = GI.features(11, 32, 64), GI.features(12, g.num_edges(), 64)
     out = _run_conv(_make_conv(norm, 64, 100, train), g, x, y, 100, 64)
     ref = {k: gold[f"{tag}.{k}"] for k in out}
-    assert_dict_close(out, ref, what=tag)
+    assert_dict_close({k: GI.sample(v) for k, v in out.items()}, ref, what=tag)
 
 
 @pytest.mark.parametrize("tag,norm,train", CONV_TAGS)
@@ -87,11 +87,9 @@ def test_conv_linegraph_d256_vs_reference_golden(golden_dir, tag, norm, train):
     g, lg, _, _ = synthetic.make_batch(batch_size=1, atoms=10, k=12, seed=5)
     xm, z = GI.features(21, g.num_edges(), 256), GI.features(22, lg.num_edges(), 256)
     out = _run_conv(_make_conv(norm, 256, 200, train), lg, xm, z, 200, 256)
-    for k in ("x_out", "gx", "g.edge_gate.weight", "g.src_gate.bias", "g.bn_edges.weight", "g.bn_nodes.bias",
-              "g.dst_update.weight"):
-        assert_close(out[k], gold[f"{tag}.{k}"], what=f"{tag}.{k}")
-    assert_close(out["y_out"][::7], gold[f"{tag}.y_out_s"], what="y_out")
-    assert_close(out["gy"][::7], gold[f"{tag}.gy_s"], what="gy")
+    for k in ("x_out", "y_out", "gx", "gy", "g.edge_gate.weight", "g.src_gate.bias", "g.bn_edges.weight",
+              "g.bn_nodes.bias", "g.dst_update.weight"):
+        assert_close(GI.sample(out[k]), gold[f"{tag}.{k}"], what=f"{tag}.{k}")
 
 
 @pytest.mark.parametrize("norm,train", [("batchnorm", True), ("layernorm", True), ("batchnorm", False)])

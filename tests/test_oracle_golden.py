@@ -52,7 +52,7 @@ def test_conv_jvasp_matches_reference_fp64(golden_dir, tag, norm, train):
     out = _conv_run(norm, train, O.OGraph(s, d_, 32), x, y, 64, 100, torch.float64)
     for k, v in out.items():
         ref = gold[f"{tag}.{k}"]
-        np.testing.assert_allclose(v.detach().numpy(), ref, rtol=1e-10, atol=1e-11, err_msg=f"{tag}.{k}")
+        np.testing.assert_allclose(GI.sample(v), ref, rtol=1e-10, atol=1e-11, err_msg=f"{tag}.{k}")
 
 
 @pytest.mark.parametrize("tag,norm,train", CONV_TAGS)
@@ -62,11 +62,9 @@ def test_conv_linegraph_d256_matches_reference(golden_dir, tag, norm, train):
     xm, z = GI.features(21, g.num_edges(), 256), GI.features(22, lg.num_edges(), 256)
     assert GI.checksum(xm, z, *lg.edges()) == int(gold["in_crc"])
     out = _conv_run(norm, train, to_oracle(lg), xm, z, 256, 200, torch.float64)
-    for k in ("x_out", "gx", "g.edge_gate.weight", "g.src_gate.bias", "g.bn_edges.weight", "g.bn_nodes.bias",
-              "g.dst_update.weight"):
-        np.testing.assert_allclose(out[k].detach().numpy(), gold[f"{tag}.{k}"], rtol=1e-5, atol=1e-6, err_msg=k)
-    np.testing.assert_allclose(out["y_out"].detach().numpy()[::7], gold[f"{tag}.y_out_s"], rtol=1e-5, atol=1e-6)
-    np.testing.assert_allclose(out["gy"].detach().numpy()[::7], gold[f"{tag}.gy_s"], rtol=1e-5, atol=1e-6)
+    for k in ("x_out", "y_out", "gx", "gy", "g.edge_gate.weight", "g.src_gate.bias", "g.bn_edges.weight",
+              "g.bn_nodes.bias", "g.dst_update.weight"):
+        np.testing.assert_allclose(GI.sample(out[k]), gold[f"{tag}.{k}"], rtol=1e-5, atol=1e-6, err_msg=k)
 
 
 def _small_cases():
